@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # our arm (CUDA kernels)
     python bench.py --impl reference --gpus N --steps K ...  # the reference's CPU path
+    python bench.py ... --dump-outputs DIR                   # also save the last timed step's outputs
 
 A "step" is one pass of the hot path over one batch of synthetic volumes:
 ``Compose([Affine, ElasticDeformation, BiasField, Blur, Noise, Gamma])`` on
@@ -54,7 +55,12 @@ def parse_args():
                     help="skip the configs[3] / configs[4] / gpu_baseline legs after the main timed region")
     ap.add_argument("--labels", action="store_true",
                     help="configs[3] shape: add an int16 LabelMap (nearest-neighbour resample) to every volume")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", type=Path,
+                    help="after the timed steps, write what the last one returned as DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
 
 
 def pipeline_spec(workload):
@@ -79,6 +85,30 @@ def synth_volumes(batch, size, pin):
         g = torch.Generator().manual_seed(1000 + b)
         torch.rand((1, size, size, size), generator=g, out=out[b])
     return out
+
+
+DUMP_BYTES = 32 << 20  # float32 voxel values written by --dump-outputs, over all images
+
+
+def dump_outputs(batch, directory):
+    """Write a step's outputs so that two builds can be compared output for output.
+
+    Per image ``<name>`` of the batch: ``<name>_affines.npy``, the (B, 4, 4) float64 affines, and
+    ``<name>.npy`` in float32: the whole (B, C, I, J, K) tensor when it fits DUMP_BYTES, else the
+    voxels at flat indices ``torch.randint(numel, (n,), generator=torch.Generator().manual_seed(0))``,
+    sorted, so that runs with the same arguments sample the same voxels."""
+    import numpy as np
+
+    directory.mkdir(parents=True, exist_ok=True)
+    per_image = DUMP_BYTES // 4 // len(batch.images)
+    for name, ib in batch.images.items():
+        data = ib.data
+        if data.numel() > per_image:
+            g = torch.Generator().manual_seed(0)
+            index = torch.randint(data.numel(), (per_image,), generator=g).sort().values
+            data = data.reshape(-1)[index.to(data.device)]
+        np.save(directory / f"{name}.npy", data.float().cpu().numpy())
+        np.save(directory / f"{name}_affines.npy", np.stack([a.numpy() for a in ib.affines]).astype(np.float64))
 
 
 # ----------------------------------------------------------------------------
@@ -240,6 +270,8 @@ def run_b200(args, rank, world, local_rank):
     launches = ops.launches() - launches0
     clocks = sampler.stop(wall_begin, wall_end) if sampler else None
     k1_ms = [s.elapsed_time(e) for s, e in k1_events]
+    if args.dump_outputs is not None and rank == 0:
+        dump_outputs(out, args.dump_outputs)
     del out
 
     # end to end through the public call with HOST buffers: pinned input ->
