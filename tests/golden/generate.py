@@ -29,7 +29,8 @@ sys.path.insert(2, str(HERE.parent))
 
 import torchio as tio  # noqa: E402  (the reference)
 
-from golden_cases import CALL_CASES, CASES, NEIGHBOUR_CASES, RESAMPLE_CASES, STAT_CASES, build_inputs  # noqa: E402
+from golden_cases import (  # noqa: E402
+    CALL_CASES, CASES, CASES_BY_NAME, NEIGHBOUR_CASES, RESAMPLE_CASES, STAT_CASES, TILE_CASE_NAMES, build_inputs)
 
 
 def _make_transform(spec):
@@ -72,18 +73,31 @@ def run_case(case):
     return arrays
 
 
+def _unchanged(path, arrays):
+    """True when ``path`` already holds exactly ``arrays`` (the zip container stamps the time of
+    writing, so rewriting identical data would still change the file)."""
+    if not path.exists():
+        return False
+    with np.load(path) as z:
+        return set(z.files) == set(arrays) and all(
+            z[k].dtype == v.dtype and np.array_equal(z[k], v) for k, v in arrays.items())
+
+
 def main():
     torch.set_num_threads(1)
     out_dir = HERE
     only = sys.argv[1] if len(sys.argv) > 1 else "all"   # "neighbours": leave the hot-path fixtures alone
     selected = {"neighbours": NEIGHBOUR_CASES, "call": CALL_CASES, "stats": STAT_CASES,
-                "resample": RESAMPLE_CASES}.get(only, CASES + NEIGHBOUR_CASES + CALL_CASES + STAT_CASES + RESAMPLE_CASES)
+                "resample": RESAMPLE_CASES, "tiles": [CASES_BY_NAME[n] for n in TILE_CASE_NAMES]}.get(
+        only, CASES + NEIGHBOUR_CASES + CALL_CASES + STAT_CASES + RESAMPLE_CASES)
     for case in selected:
         arrays = run_case(case)
         path = out_dir / f"{case['name']}.npz"
-        np.savez_compressed(path, **arrays)
+        state = "unchanged" if _unchanged(path, arrays) else "written"
+        if state == "written":
+            np.savez_compressed(path, **arrays)
         size = path.stat().st_size / 1024
-        print(f"{case['name']:40s} {size:8.1f} KiB")
+        print(f"{case['name']:40s} {size:8.1f} KiB  {state}")
 
 
 if __name__ == "__main__":

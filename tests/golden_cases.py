@@ -186,6 +186,26 @@ CASES = [
                     ("Blur", {"std": (0.0, 2.0)}),
                     ("Noise", {"std": (0.0, 0.25)}),
                     ("Gamma", {"log_gamma": (-0.3, 0.3)})]),
+    # ---- K1 tile kernels (TMA boxes): K * element size a multiple of 16 bytes and at least one
+    # full 16^3 output tile per axis, so most tiles walk the staged box instead of the general column
+    dict(name="elastic_aniso_tiles", seed=131, shape=(40, 36, 48), batch=2,
+         spacing=(0.8, 1.1, 2.0), origin=(2.0, -3.0, 1.0),
+         images={"t1": "scalar", "seg": "uint8"},
+         transform=("ElasticDeformation", {"max_displacement": (3.0, 5.0, 6.0),
+                                           "num_control_points": (7, 6, 8)})),
+    # control cells of 5.2 / 6.5 / 5.25 voxels, the densest grid whose every tile the bounds pre-pass
+    # still accepts (it gives up beyond two cell crossings per 16-voxel tile axis): the walk changes
+    # cell inside a 16-plane tile two or three times, sometimes between the planes of one pair
+    dict(name="elastic_dense_grid_tiles", seed=132, shape=(48, 40, 64), batch=1,
+         spacing=(1.0, 1.0, 2.0), images={"t1": "scalar", "seg": "int16"},
+         transform=("ElasticDeformation", {"max_displacement": 1.5,
+                                           "num_control_points": (10, 7, 13), "locked_borders": 0})),
+    # half-voxel translations: fill decisions exactly on the mask threshold of 0.5
+    dict(name="affine_half_voxel_fill", seed=133, shape=(40, 36, 48), batch=1, channels=2,
+         images={"t1": "scalar", "seg": "int16"},
+         transform=("Affine", {"scales": (1.0, 1.0), "degrees": (0.0, 0.0),
+                               "translation": (0.5, 0.5, -1.5, -1.5, 2.5, 2.5),
+                               "default_pad_value": -1.0, "default_pad_label": 7})),
 ]
 
 # ---- index-remap neighbours of the chain (SURVEY §8 f-3): Flip / Crop / Pad ----------
@@ -298,7 +318,23 @@ RESAMPLE_CASES = [
     dict(name="label_pv_onehot_nearest", seed=121, shape=(16, 14, 12), batch=2,
          images={"seg": "uint8"},
          transform=("Affine", {**_AFF, "label_interpolation": "label", "one_hot_label_interpolation": "nearest"})),
+    # ---- K1 tile kernels on target grids (see the tile cases of CASES)
+    # a permuted, flipped target grid (like _TARGET_AFFINE) of full 16^3 tiles inside the input's field of view
+    dict(name="spatial_target_tiles", seed=134, shape=(40, 36, 48), batch=2, spacing=(1.2, 0.9, 1.5),
+         images={"t1": "scalar", "seg": "int16"},
+         transform=("Spatial", {**_AFF, "max_displacement": (1.0, 2.5), "num_control_points": 6,
+                                "target": ((32, 32, 32), [[0.0, -1.3, 0.0, 44.0], [1.1, 0.0, 0.0, -1.0],
+                                                          [0.0, 0.0, 1.6, 8.0], [0.0, 0.0, 0.0, 1.0]])})),
+    dict(name="resample_down_tiles", seed=135, shape=(48, 48, 64), batch=2, spacing=(0.9, 0.9, 1.0),
+         images={"t1": "scalar", "seg": "uint8"}, transform=("Resample", {"target": (1.35, 1.35, 2.0)})),
+    dict(name="label_pv_aniso_tiles", seed=136, shape=(40, 36, 48), batch=2, spacing=(0.8, 1.1, 2.0),
+         images={"seg": "int16"},
+         transform=("Spatial", {**_AFF, "max_displacement": (1.0, 3.0), "num_control_points": 7,
+                                "label_interpolation": "label", "default_pad_label": 9})),
 ]
+# the cases above made for the K1 tile kernels (``generate.py tiles`` writes only these)
+TILE_CASE_NAMES = ("elastic_aniso_tiles", "elastic_dense_grid_tiles", "affine_half_voxel_fill",
+                   "spatial_target_tiles", "resample_down_tiles", "label_pv_aniso_tiles")
 
 # ---- BASELINE.json's own volume size: 256^3 (configs[1] and configs[2], two elements) ----------
 # The reference's full outputs are too large to commit (64 MiB per volume): the fixture keeps
